@@ -1,4 +1,4 @@
-"""Reference arm of bench.py: the UNMODIFIED intel/MLSL (baseline/_ref, built by baseline/install_ref.sh) running the
+"""Reference arm of bench.py: the UNMODIFIED intel/MLSL (oracle/_ref, built by oracle/install_ref.sh) running the
 same metric - fp32 SUM all-reduce bus bandwidth of the headline message through its own public API
 (Environment::Alloc + Distribution::AllReduce + Environment::Wait, stock "process" mode, N MPI ranks on this node
 launched by its bundled mpiexec.hydra).  The reference is a CPU library: its buffers live in host memory, so the
@@ -9,7 +9,7 @@ import os
 import subprocess
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF = os.path.join(HERE, "_ref")
+REF = os.path.join(os.path.dirname(HERE), "oracle", "_ref")
 
 
 def _env(overrides=None):
@@ -37,7 +37,7 @@ def _env(overrides=None):
 def _run(nranks, minb, maxb, iters, warm, factor, timeout):
     exe = os.path.join(REF, "bin", "ref_allreduce_bench")
     if not os.path.exists(exe):
-        raise RuntimeError("baseline/_ref is not installed (run baseline/install_ref.sh)")
+        raise RuntimeError("oracle/_ref is not installed (run oracle/install_ref.sh <reference checkout>)")
     hydra = os.path.join(REF, "mpirt", "bin", "mpiexec.hydra")
     tail = [exe, str(minb), str(maxb), str(iters), str(warm), str(factor)]
     res = None
@@ -84,7 +84,7 @@ def run(n_gpus, steps, warmup, headline_bytes):
                    "parallelism": "dp%d" % n, "message_bytes": headline_bytes,
                    "api": "MLSL::Distribution::AllReduce + Environment::Wait (intel/MLSL process mode, Intel MPI shm)",
                    "device": "CPU (the reference has no GPU path); host-timed, max over ranks",
-                   "launcher": "baseline/_ref/mpirt/bin/mpiexec.hydra -n %d" % n},
+                   "launcher": "oracle/_ref/mpirt/bin/mpiexec.hydra -n %d" % n},
         "e2e": {"value": round(value, 4), "unit": "GB/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0,
                 "note": "buffers are host resident: the measured value already is end to end"},
         "gpu_launches": 0, "sweep": sweep,

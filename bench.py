@@ -3,7 +3,8 @@
 device-timed, max over ranks").
 
     python bench.py --gpus N --steps K --warmup W            # ours (N>1: launched by torchrun, one rank per GPU)
-    python bench.py --impl reference --gpus N ...            # the unmodified reference (CPU/MPI library) from baseline/_ref
+    python bench.py --impl reference --gpus N ...            # the unmodified reference (CPU/MPI library) from oracle/_ref
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's output to DIR/*.npy
 
 One "step" = one fp32 SUM all-reduce of the headline message (1 GiB per rank, out of place, with the 1/N averaging
 scale fused into the kernel) through the public API (mlsl_b200.allreduce -> Distribution::AllReduceEx ->
@@ -43,6 +44,7 @@ def parse_args():
     ap.add_argument("--nccl", action="store_true", help="(default at N > 1) also time torch.distributed (NCCL) all_reduce")
     ap.add_argument("--no-nccl", action="store_true", help="skip the NCCL comparison")
     ap.add_argument("--compress", action="store_true", help="headline through the fp8-compressed transport")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the output of the last timed step as DIR/<name>.npy")
     return ap.parse_args()
 
 
@@ -159,6 +161,24 @@ def roofline(world, S, ms, nvls):
     return {"frac": round(algbw * busbw_factor(world) / LINK_GBS, 4), "ceiling": "peer-to-peer two-shot: busbw <= %.0f GB/s (measured link; nominal 900)" % LINK_GBS}
 
 
+DUMP_ELEMS = 1 << 22     # 16 MiB of float32 per array: larger outputs are dumped as a fixed, seeded sample
+
+
+def dump_outputs(d, arrays):
+    """--dump-outputs: every array as <d>/<name>.npy in float32.  An array of more than DUMP_ELEMS elements is sampled at
+    the same sorted, seeded indices on every run, so that the dumps of two builds compare element for element."""
+    import numpy as np
+    import torch
+
+    os.makedirs(d, exist_ok=True)
+    for name, t in arrays.items():
+        flat = t.reshape(-1)
+        if flat.numel() > DUMP_ELEMS:
+            idx = np.sort(np.random.default_rng(0).integers(0, flat.numel(), DUMP_ELEMS))
+            flat = flat[torch.from_numpy(idx).to(flat.device)]
+        np.save(os.path.join(d, name + ".npy"), flat.float().cpu().numpy())
+
+
 def run_ours(args):
     import torch
 
@@ -260,6 +280,8 @@ def run_ours(args):
     ms, h0, h1 = timed(lambda: step_device(x, y, n), args.steps, warm, want_window=True)
     clocks = sampler.stop(h0, h1) if sampler else None
     torch.cuda.synchronize()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"allreduce_out": y[:n]})
     y_bad = verify(y, n, *( (0.08, 0.08) if args.compress else (2e-5, 2e-5)))
     ok = y_bad == 0
     describe = env.describe_backend()
